@@ -14,7 +14,6 @@ GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA (sm_100a) device; run with `-m gpu` on the B200 box")
-    config.addinivalue_line("markers", "reference: needs the read-only reference tree at /root/reference (build container only)")
 
 
 def load_npz(name):

@@ -447,11 +447,100 @@ def gen_vad():
     print("vad cases", [(len(c["probs"]), len(c["timestamps"])) for c in out])
 
 
+def sample_array(out, key, a, n=128, top_k=0):
+    """Store a fixed sample of ``a``: its shape, ``n`` flat positions drawn with a fixed seed and (``top_k`` > 0, for
+    probabilities [..., V]) every row's argmax and ``top_k`` largest entries, where fp32 differences are largest.
+    Keeps a chunk's [T, 4233] posteriors and its caches to a few KB each."""
+    a = np.ascontiguousarray(np.asarray(a, np.float32))
+    flat = a.reshape(-1)
+    idx = np.arange(flat.size) if flat.size <= n else np.random.default_rng(len(out)).choice(flat.size, n, replace=False)
+    if top_k:
+        rows = a.reshape(-1, a.shape[-1])
+        top = np.argsort(-rows, axis=1, kind="stable")[:, :top_k]
+        idx = np.concatenate([idx, (np.arange(rows.shape[0])[:, None] * rows.shape[1] + top).reshape(-1)])
+        out[key + "/ids"] = rows.argmax(1).astype(np.int32)
+    idx = np.unique(idx)
+    out[key + "/shape"] = np.asarray(a.shape, np.int64)
+    out[key + "/idx"] = idx.astype(np.int32)
+    out[key + "/val"] = flat[idx]
+
+
+def gen_reference_chunks(tmp):
+    """The reference's featurizer, the Conformer's whole-utterance forward and the chunk-by-chunk forward of every
+    streaming model (posteriors and both caches after each chunk, the last chunk short), sampled by ``sample_array``.
+    Frozen so that tests/test_oracle_vs_reference.py can check the oracle's chunk paths without the reference."""
+    from masr.data_utils.audio import AudioSegment
+    from masr.data_utils.featurizer.audio_featurizer import AudioFeaturizer
+    from masr.model_utils.deepspeech2.model import DeepSpeech2Model
+    from masr.model_utils.efficient_conformer.model import EfficientConformerModel
+    from masr.model_utils.squeezeformer.model import SqueezeformerModel
+    from oracle import fbank as ob
+    out = {}
+    af = AudioFeaturizer(feature_method="fbank", n_mels=80, sample_rate=16000, use_dB_normalization=True, target_dB=-20)
+    for kind, seed, n in [("noise", 5, 20000), ("speech", 6, 33333)]:
+        feat = af.featurize(AudioSegment.from_ndarray(make_audio(kind, seed, n), 16000))
+        sample_array(out, f"fbank/{kind}_{seed}", feat, n=1024)
+    pcm = (make_audio("speech", 7, 8000) * 20000).astype(np.int16)
+    sample_array(out, "fbank/pcm_speech_7", af.featurize(AudioSegment.from_pcm_bytes(pcm.tobytes())), n=1024)
+
+    def featurize(kind, seed, n):
+        return torch.from_numpy(ob.featurize(make_audio(kind, seed, n)))[None]
+
+    def build(cls, yml, sdn, strict=False, model_conf=True):
+        cfg = yaml.safe_load(open(os.path.join(ref_shims.REFERENCE_ROOT, "configs", yml), encoding="utf-8"))
+        mi = os.path.join(tmp, "mi.json")
+        synth.write_mean_istd(mi, 0)
+        m = cls(input_dim=80, vocab_size=V, mean_istd_path=mi, streaming=True, encoder_conf=cfg["encoder_conf"],
+                decoder_conf=cfg["decoder_conf"], **(cfg["model_conf"] if model_conf else {})).eval()
+        m.load_state_dict(synth.to_torch(sdn), strict=strict)
+        return m
+
+    def attention_chunks(name, m, feat, first_len):
+        att = torch.zeros(0, 0, 0, 0)
+        cnn = torch.zeros(0, 0, 0, 0)
+        off = 0
+        nf = feat.shape[1]
+        for i, cur in enumerate(range(0, nf - first_len + 1, 64)):
+            pr, att, cnn = m.get_encoder_out_chunk(feat[:, cur:min(cur + 67, nf)], off, -16, att, cnn)
+            off += pr.shape[1]
+            sample_array(out, f"{name}/{i}/probs", pr, top_k=4)
+            sample_array(out, f"{name}/{i}/att", att)
+            sample_array(out, f"{name}/{i}/cnn", cnn)
+
+    with torch.no_grad():
+        m, _, _ = build_reference_model(tmp, True, 0)
+        feat = featurize("speech", 8, 16000 * 3)
+        sample_array(out, "conformer/full", m.get_encoder_out(feat, torch.tensor([feat.shape[1]])), n=1024, top_k=8)
+        attention_chunks("conformer", m, feat, 67)
+        m = build(SqueezeformerModel, "squeezeformer.yml", synth.squeezeformer_state_dict(0, V, streaming=True))
+        attention_chunks("squeezeformer", m, featurize("speech", 9, 16000 * 3 + 4000), 7)
+        m = build(EfficientConformerModel, "efficient_conformer.yml", synth.efficient_conformer_state_dict(0, V))
+        attention_chunks("efficient", m, featurize("speech", 13, 16000 * 3 + 4000), 7)
+        m = build(DeepSpeech2Model, "deepspeech2.yml", synth.deepspeech2_state_dict(0, V, streaming=True), strict=True,
+                  model_conf=False)
+        feat = featurize("speech", 14, 16000 * 3 + 4000)
+        h = torch.zeros(0, 0, 0, 0)
+        c = torch.zeros(0, 0, 0, 0)
+        nf = feat.shape[1]
+        for i, cur in enumerate(range(0, nf - 7 + 1, 64)):
+            ch = feat[:, cur:min(cur + 67, nf)]
+            pr, lens, h, c = m.get_encoder_out_chunk(ch, torch.tensor([ch.shape[1]]), h, c)
+            out[f"deepspeech2/{i}/len"] = lens.numpy().astype(np.int64)
+            sample_array(out, f"deepspeech2/{i}/probs", pr[0], top_k=4)
+            sample_array(out, f"deepspeech2/{i}/h", h.reshape(-1))
+            sample_array(out, f"deepspeech2/{i}/c", c.reshape(-1))
+    np.savez_compressed(os.path.join(HERE, "reference_chunks_golden.npz"), **out)
+    print("reference_chunks_golden.npz", len(out), "arrays")
+
+
 if __name__ == "__main__":
     torch.set_num_threads(8)
     with tempfile.TemporaryDirectory() as tmp:
         which = sys.argv[1:] or ["fbank", "encoder", "predictor", "efficient", "squeezeformer", "deepspeech2",
-                                  "predictor_squeezeformer", "predictor_efficient", "predictor_deepspeech2", "vad"]
+                                  "predictor_squeezeformer", "predictor_efficient", "predictor_deepspeech2", "vad",
+                                  "reference_chunks"]
+        if "reference_chunks" in which:
+            gen_reference_chunks(tmp)
         if "deepspeech2" in which:
             gen_deepspeech2(tmp)
         if "squeezeformer" in which:

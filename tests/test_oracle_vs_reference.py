@@ -1,174 +1,112 @@
-"""CPU, build container only: the oracle against the live, unmodified reference (skipped where
-/root/reference is absent, e.g. on the GPU box)."""
-import json
+"""CPU: the oracle against the unmodified reference's featurizer, whole-utterance Conformer forward and chunk-by-chunk
+forward of every streaming model, frozen by tests/golden/make_golden.py as fixed samples of each output
+(tests/golden/reference_chunks_golden.npz)."""
 import os
 
 import numpy as np
 import pytest
 import torch
 
-from conftest import make_audio, synth_weights
+from conftest import GOLDEN, make_audio, synth_weights
 from masr_b200 import synth
-from oracle import conformer as oc, fbank as ob, ref_shims
+from oracle import conformer as oc, fbank as ob
 
-pytestmark = [pytest.mark.reference,
-              pytest.mark.skipif(not ref_shims.reference_available(), reason="reference tree not present")]
+# The frozen outputs were computed by the reference on one CPU.  On another, torch's fp32 CPU kernels (MKL, oneDNN, ATen)
+# sum in another order: the posteriors move by up to 2.5e-6 and the Conformer's caches by up to 2.2e-6 (measured with
+# the kernels limited to AVX2, to baseline x86-64 and to MKL's compatible mode).  Where the oracle and the reference run
+# the same ops on the same CPU they agree bit for bit.
+PROB_TOL = 5e-6
 
 
 @pytest.fixture(scope="module")
-def ref_model(tmp_path_factory):
-    ref_shims.install()
-    import yaml
-    from masr.model_utils.conformer.model import ConformerModel
-    tmp = tmp_path_factory.mktemp("ref")
-    cfg = yaml.safe_load(open(os.path.join(ref_shims.REFERENCE_ROOT, "configs", "conformer.yml"), encoding="utf-8"))
-    mi = str(tmp / "mi.json")
-    synth.write_mean_istd(mi, 0)
-    m = ConformerModel(input_dim=80, vocab_size=synth.DEFAULT_VOCAB_SIZE, mean_istd_path=mi, streaming=True,
-                       encoder_conf=cfg["encoder_conf"], decoder_conf=cfg["decoder_conf"], **cfg["model_conf"]).eval()
-    m.load_state_dict(synth.to_torch(synth_weights(0)), strict=False)
-    return m
+def golden():
+    return np.load(os.path.join(GOLDEN, "reference_chunks_golden.npz"))
 
 
-def test_featurizer_matches(ref_model):
-    from masr.data_utils.audio import AudioSegment
-    from masr.data_utils.featurizer.audio_featurizer import AudioFeaturizer
-    af = AudioFeaturizer(feature_method="fbank", n_mels=80, sample_rate=16000, use_dB_normalization=True, target_dB=-20)
+def close(z, key, got, tol):
+    """``got`` (full array) against the stored sample of the reference's array ``key``: same shape, same per-frame
+    argmax (posteriors), sampled entries within ``tol``."""
+    got = np.asarray(got, np.float32)
+    assert got.shape == tuple(z[key + "/shape"]), key
+    if key + "/ids" in z.files:
+        assert np.array_equal(got.reshape(-1, got.shape[-1]).argmax(1), z[key + "/ids"]), key
+    err = np.abs(got.reshape(-1)[z[key + "/idx"]] - z[key + "/val"]).max()
+    assert err < tol, (key, float(err))
+
+
+def test_featurizer_matches(golden):
     for kind, seed, n in [("noise", 5, 20000), ("speech", 6, 33333)]:
-        x = make_audio(kind, seed, n)
-        ref = af.featurize(AudioSegment.from_ndarray(x.copy(), 16000))
-        assert np.abs(ob.featurize(x.copy()) - ref).max() < 5e-4
+        close(golden, f"fbank/{kind}_{seed}", ob.featurize(make_audio(kind, seed, n)), 5e-4)
     pcm = (make_audio("speech", 7, 8000) * 20000).astype(np.int16)
-    ref = af.featurize(AudioSegment.from_pcm_bytes(pcm.tobytes()))
-    assert np.abs(ob.featurize(ob.pcm_bytes_to_float32(pcm.tobytes())) - ref).max() < 5e-4
+    close(golden, "fbank/pcm_speech_7", ob.featurize(ob.pcm_bytes_to_float32(pcm.tobytes())), 5e-4)
 
 
-def test_full_and_chunk_forward_match(ref_model):
+def featurize(kind, seed, n):
+    return torch.from_numpy(ob.featurize(make_audio(kind, seed, n)))[None]
+
+
+def check_attention_chunks(z, name, encode_chunk, st, feat, first_len, cache_tol):
+    """Feed ``feat`` in 67-frame windows every 64 frames (the reference's ``predict_stream`` windows, the last one short
+    unless ``first_len`` == 67) and compare the posteriors and both caches after every chunk."""
+    nf = feat.shape[1]
+    n = 0
+    for i, cur in enumerate(range(0, nf - first_len + 1, 64)):
+        pm = encode_chunk(feat[:, cur:min(cur + 67, nf)], st)
+        close(z, f"{name}/{i}/probs", pm, PROB_TOL)
+        close(z, f"{name}/{i}/att", st.att_cache, cache_tol)
+        close(z, f"{name}/{i}/cnn", st.cnn_cache, cache_tol)
+        n += 1
+    assert f"{name}/{n}/probs/shape" not in z.files and n > 1
+
+
+def test_full_and_chunk_forward_match(golden):
     sd = synth.to_torch(synth_weights(0))
     cfg = oc.ConformerConfig()
-    feat = torch.from_numpy(ob.featurize(make_audio("speech", 8, 16000 * 3)))[None]
+    feat = featurize("speech", 8, 16000 * 3)
     with torch.no_grad():
-        ref = ref_model.get_encoder_out(feat, torch.tensor([feat.shape[1]]))
-        got = oc.get_encoder_out(sd, cfg, feat)
-        assert (ref - got).abs().max().item() < 1e-6
-        st = oc.ChunkState()
-        att = torch.zeros(0, 0, 0, 0)
-        cnn = torch.zeros(0, 0, 0, 0)
-        off = 0
-        for cur in range(0, feat.shape[1] - 67 + 1, 64):
-            ch = feat[:, cur:cur + 67]
-            pr, att, cnn = ref_model.get_encoder_out_chunk(ch, off, -16, att, cnn)
-            off += pr.shape[1]
-            pm = oc.get_encoder_out_chunk(sd, cfg, ch, st, -16)
-            assert (pr - pm).abs().max().item() < 1e-6
-            assert (att - st.att_cache).abs().max().item() < 1e-6
-            assert (cnn - st.cnn_cache).abs().max().item() < 1e-6
+        close(golden, "conformer/full", oc.get_encoder_out(sd, cfg, feat), PROB_TOL)
+        check_attention_chunks(golden, "conformer", lambda ch, st: oc.get_encoder_out_chunk(sd, cfg, ch, st, -16),
+                               oc.ChunkState(), feat, 67, 1e-5)
 
 
-def test_squeezeformer_chunk_forward_matches():
-    """oracle/squeezeformer.get_encoder_out_chunk against the live reference's TorchScript-able chunk method, chunk by
-    chunk (probabilities and both caches), including a short final chunk."""
-    ref_shims.install()
-    import tempfile
-    import yaml
-    from masr.model_utils.squeezeformer.model import SqueezeformerModel
+def test_squeezeformer_chunk_forward_matches(golden):
+    """oracle/squeezeformer.get_encoder_out_chunk against the reference's TorchScript-able chunk method, chunk by chunk
+    (probabilities and both caches), including a short final chunk."""
     from oracle import squeezeformer as osq
-    cfg_y = yaml.safe_load(open(os.path.join(ref_shims.REFERENCE_ROOT, "configs", "squeezeformer.yml"), encoding="utf-8"))
-    with tempfile.TemporaryDirectory() as tmp:
-        mi = os.path.join(tmp, "mi.json")
-        synth.write_mean_istd(mi, 0)
-        m = SqueezeformerModel(input_dim=80, vocab_size=synth.DEFAULT_VOCAB_SIZE, mean_istd_path=mi, streaming=True,
-                               encoder_conf=cfg_y["encoder_conf"], decoder_conf=cfg_y["decoder_conf"], **cfg_y["model_conf"]).eval()
-    sdn = synth.squeezeformer_state_dict(0, streaming=True)
-    m.load_state_dict(synth.to_torch(sdn), strict=False)
-    sd = synth.to_torch(sdn)
+    sd = synth.to_torch(synth.squeezeformer_state_dict(0, streaming=True))
     cfg = osq.SqueezeformerConfig(causal=True)
-    feat = torch.from_numpy(ob.featurize(make_audio("speech", 9, 16000 * 3 + 4000)))[None]
     with torch.no_grad():
-        st = osq.ChunkState()
-        att = torch.zeros(0, 0, 0, 0)
-        cnn = torch.zeros(0, 0, 0, 0)
-        off = 0
-        nf = feat.shape[1]
-        for cur in range(0, nf - 7 + 1, 64):
-            ch = feat[:, cur:min(cur + 67, nf)]
-            pr, att, cnn = m.get_encoder_out_chunk(ch, off, -16, att, cnn)
-            off += pr.shape[1]
-            pm = osq.get_encoder_out_chunk(sd, cfg, ch, st, -16)
-            assert pr.shape == pm.shape
-            assert torch.equal(pr.argmax(-1), pm.argmax(-1))
-            assert (pr - pm).abs().max().item() < 5e-6          # fp32 summation-order noise (different operand strides)
-            assert att.shape == st.att_cache.shape and (att - st.att_cache).abs().max().item() < 2e-5
-            assert cnn.shape == st.cnn_cache.shape and (cnn - st.cnn_cache).abs().max().item() < 2e-5
+        check_attention_chunks(golden, "squeezeformer", lambda ch, st: osq.get_encoder_out_chunk(sd, cfg, ch, st, -16),
+                               osq.ChunkState(), featurize("speech", 9, 16000 * 3 + 4000), 7, 2e-5)
 
 
-def test_efficient_conformer_chunk_forward_matches():
-    """oracle/efficient_conformer.get_encoder_out_chunk against the live reference, chunk by chunk (probabilities and
+def test_efficient_conformer_chunk_forward_matches(golden):
+    """oracle/efficient_conformer.get_encoder_out_chunk against the reference, chunk by chunk (probabilities and
     both caches), including a short final chunk."""
-    ref_shims.install()
-    import tempfile
-    import yaml
-    from masr.model_utils.efficient_conformer.model import EfficientConformerModel
     from oracle import efficient_conformer as oe
-    cfg_y = yaml.safe_load(open(os.path.join(ref_shims.REFERENCE_ROOT, "configs", "efficient_conformer.yml"), encoding="utf-8"))
-    with tempfile.TemporaryDirectory() as tmp:
-        mi = os.path.join(tmp, "mi.json")
-        synth.write_mean_istd(mi, 0)
-        m = EfficientConformerModel(input_dim=80, vocab_size=synth.DEFAULT_VOCAB_SIZE, mean_istd_path=mi, streaming=True,
-                                    encoder_conf=cfg_y["encoder_conf"], decoder_conf=cfg_y["decoder_conf"], **cfg_y["model_conf"]).eval()
-    sdn = synth.efficient_conformer_state_dict(0)
-    m.load_state_dict(synth.to_torch(sdn), strict=False)
-    sd = synth.to_torch(sdn)
+    sd = synth.to_torch(synth.efficient_conformer_state_dict(0))
     cfg = oe.EfficientConfig()
-    feat = torch.from_numpy(ob.featurize(make_audio("speech", 13, 16000 * 3 + 4000)))[None]
     with torch.no_grad():
-        st = oe.ChunkState()
-        att = torch.zeros(0, 0, 0, 0)
-        cnn = torch.zeros(0, 0, 0, 0)
-        off = 0
-        nf = feat.shape[1]
-        for cur in range(0, nf - 7 + 1, 64):
-            ch = feat[:, cur:min(cur + 67, nf)]
-            pr, att, cnn = m.get_encoder_out_chunk(ch, off, -16, att, cnn)
-            off += pr.shape[1]
-            pm = oe.get_encoder_out_chunk(sd, cfg, ch, st, -16)
-            assert pr.shape == pm.shape
-            assert torch.equal(pr.argmax(-1), pm.argmax(-1))
-            assert (pr - pm).abs().max().item() < 5e-6
-            assert att.shape == st.att_cache.shape and (att - st.att_cache).abs().max().item() < 2e-5
-            assert cnn.shape == st.cnn_cache.shape and (cnn - st.cnn_cache).abs().max().item() < 2e-5
+        check_attention_chunks(golden, "efficient", lambda ch, st: oe.get_encoder_out_chunk(sd, cfg, ch, st, -16),
+                               oe.ChunkState(), featurize("speech", 13, 16000 * 3 + 4000), 7, 2e-5)
 
 
-def test_deepspeech2_chunk_forward_matches():
-    """oracle/deepspeech2.get_encoder_out with a carried (h, c) state against the live reference's
+def test_deepspeech2_chunk_forward_matches(golden):
+    """oracle/deepspeech2.get_encoder_out with a carried (h, c) state against the reference's
     ``get_encoder_out_chunk`` (deepspeech2/model.py:70-77), window by window."""
-    ref_shims.install()
-    import tempfile
-    import yaml
-    from masr.model_utils.deepspeech2.model import DeepSpeech2Model
     from oracle import deepspeech2 as od
-    cfg_y = yaml.safe_load(open(os.path.join(ref_shims.REFERENCE_ROOT, "configs", "deepspeech2.yml"), encoding="utf-8"))
-    with tempfile.TemporaryDirectory() as tmp:
-        mi = os.path.join(tmp, "mi.json")
-        synth.write_mean_istd(mi, 0)
-        m = DeepSpeech2Model(input_dim=80, vocab_size=synth.DEFAULT_VOCAB_SIZE, mean_istd_path=mi, streaming=True,
-                             encoder_conf=cfg_y["encoder_conf"], decoder_conf=cfg_y["decoder_conf"]).eval()
-    sdn = synth.deepspeech2_state_dict(0, streaming=True)
-    m.load_state_dict(synth.to_torch(sdn), strict=True)
-    sd = synth.to_torch(sdn)
+    sd = synth.to_torch(synth.deepspeech2_state_dict(0, streaming=True))
     cfg = od.DS2Config(bidirectional=False)
-    feat = torch.from_numpy(ob.featurize(make_audio("speech", 14, 16000 * 3 + 4000)))[None]
+    feat = featurize("speech", 14, 16000 * 3 + 4000)
+    nf = feat.shape[1]
+    state = None
+    n = 0
     with torch.no_grad():
-        h = torch.zeros(0, 0, 0, 0)
-        c = torch.zeros(0, 0, 0, 0)
-        state = None
-        nf = feat.shape[1]
-        for cur in range(0, nf - 7 + 1, 64):
-            ch = feat[:, cur:min(cur + 67, nf)]
-            pr, lens, h, c = m.get_encoder_out_chunk(ch, torch.tensor([ch.shape[1]]), h, c)
-            pm, state = od.get_encoder_out(sd, cfg, ch, state)
-            assert pr.shape[1] == pm.shape[0] == int(lens[0])
-            assert torch.equal(pr[0].argmax(-1), pm.argmax(-1))
-            assert (pr[0] - pm).abs().max().item() < 5e-6
-            assert (h.reshape(-1) - state[0].reshape(-1)).abs().max().item() < 2e-5
-            assert (c.reshape(-1) - state[1].reshape(-1)).abs().max().item() < 2e-5
+        for i, cur in enumerate(range(0, nf - 7 + 1, 64)):
+            pm, state = od.get_encoder_out(sd, cfg, feat[:, cur:min(cur + 67, nf)], state)
+            assert pm.shape[0] == int(golden[f"deepspeech2/{i}/len"][0])
+            close(golden, f"deepspeech2/{i}/probs", pm, PROB_TOL)
+            close(golden, f"deepspeech2/{i}/h", state[0].reshape(-1), 2e-5)
+            close(golden, f"deepspeech2/{i}/c", state[1].reshape(-1), 2e-5)
+            n += 1
+    assert f"deepspeech2/{n}/len" not in golden.files and n > 1
